@@ -2,6 +2,7 @@
 """bench.py — task x worker cost evaluations per second on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg1..cfg5]
+                    [--dump-outputs DIR]
 
 One *step* is one management pass (pm_match: cost-matrix build -> argmin ->
 resolution sweep) over one synthetic swarm.  N=1 workload: BASELINE configs[2],
@@ -19,6 +20,10 @@ goes through the C ABI with host (pinned) tables: H2D of asks+workers and D2H of
 the assignment inside the timed region.  `--impl reference` times the CPU
 oracle (the reference's scheduler restated; the Rust reference cannot be built
 here) on the box's host cores on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step computed, as DIR/<name>.npy
+in float64 (every value exact), so that two builds can be compared output for
+output on the same seeded inputs; see dump_outputs().
 """
 from __future__ import annotations
 
@@ -49,6 +54,30 @@ WORKLOADS = {
     "cfg5": (1_000_000, 1_000_000, "skewed", "1M asks x 1M workers per GPU (1M x 8M over 8 GPUs), Zipf(1.1) worker prices, 10% infeasible asks"),
 }
 PRICES = {"cfg3": "loguniform", "cfg5": "zipf"}
+DUMP_BYTES = 64_000_000         # --dump-outputs: bytes written at most, .npy headers included
+DUMP_SEED = 0xB2000004          # positions kept when the outputs are larger than that
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write each integer array as out_dir/<name>.npy in float64, which holds every u32 / i32 value exactly.  When the
+    whole would exceed `budget`, every array longer than its share keeps the same seeded positions from run to run
+    (the positions go to <name>_index.npy), so two runs on the same inputs stay comparable element for element."""
+    arrays = dict(arrays)
+    if sum(a.size for a in arrays.values()) * 8 + 128 * len(arrays) > budget:
+        share = (budget - 2 * 128 * len(arrays)) // 8 // (2 * len(arrays))     # values + positions per array
+        for name, a in list(arrays.items()):
+            if a.size > share:
+                idx = np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, share, replace=False))
+                arrays[name], arrays[name + "_index"] = a[idx], idx
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a).astype(np.float64))
+
+
+def split_best(best):
+    """Packed cost<<32 | worker keys as two arrays: float64 holds each half exactly, but not the packed int64."""
+    best = np.asarray(best, dtype=np.int64)
+    return {"ask_best_cost": best >> 32, "ask_best_worker": best & 0xFFFFFFFF}
 
 
 def host_cpus():
@@ -188,15 +217,19 @@ def run_reference(args):
 
     def step():
         return orc.soa_eval_matrix(w.a, w.b, a.asks, a.opts, bits, words, t0, t0 + sample_rows, 0, W,
-                                   threads=cores, want_rows=True, want_cols=True)["evals"]
+                                   threads=cores, want_rows=True, want_cols=True)
 
     for _ in range(args.warmup):
         step()
     t_start = time.perf_counter()
     evals = 0
     for _ in range(args.steps):
-        evals += step()
+        last = step()
+        evals += last["evals"]
     dt = time.perf_counter() - t_start
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**split_best(last["row_best"]), "ask_count": last["row_count"],
+                                         "worker_first_ask": last["col_first"]})
     value = evals / dt
     # the faithful loop (string/AoS, re-filter per group) on a small sample, single thread
     faithful = faithful_sample(orc, w, a)
@@ -335,7 +368,13 @@ def run_ours(args):
             ms = float(tms.item())
         evals_per_step = T * W
         value = evals_per_step * args.steps / (ms * 1e-3)
-        groups_formed = int(eng.fetch().n_groups)
+        last = eng.fetch()          # the last timed pass's result; every rank holds the same one
+        groups_formed = int(last.n_groups)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {
+                "worker_group": last.worker_group, "worker_ask": last.worker_ask, "group_ask": last.group_ask,
+                "group_off": last.group_off, "group_members": last.group_members, **split_best(last.ask_best),
+                "ask_count": last.ask_count})
 
         # ---- e2e: host tables in pinned memory -> H2D -> match -> D2H, all inside the timed region
         lo = rank * Wg if world > 1 else 0
@@ -518,7 +557,11 @@ def main():
                     help="distinct worker model strings (0: the 16-entry catalogue; > 31 selects the wide-catalogue kernel variants)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", dest="no_extras", action="store_true", help="skip the fused_lean / auction sub-records")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step returned as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload is None:
         args.workload = "cfg3" if args.gpus <= 1 else "cfg5"
     if args.warmup < 3 and args.impl == "ours":

@@ -4,7 +4,7 @@
   pm_match_local; the three exchange buffers are merged the way the collective merges them (concatenate / min / sum)
   and every engine runs pm_match_finish.  Groups must equal the unsharded engine's and the CPU oracle's.
 * Two or more GPUs in one process (pm_multi: NCCL all-gather inside the library): same check.  Skipped on a
-  one-GPU box; `gpurun --gpus 2` runs it.
+  machine with one GPU.
 """
 import numpy as np
 import pytest
@@ -115,7 +115,7 @@ def test_multi_engine_in_one_process(mode, sizes):
     """pm_multi on every visible GPU: NCCL all-gather inside the library, result on device 0 == oracle."""
     n = _n_devices()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     w, a, t = tables(500, 40003, group_sizes=sizes, seed_shift=23)
     prox = (mode & 0xFF) == abi.PM_MODE_PROXIMITY
     og = orc.soa_form_groups(t["wa"], t["wb"], t["asks"], t["opts"], t["bits"], t["words"], addr_rank=None,
