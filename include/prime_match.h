@@ -246,7 +246,8 @@ enum pm_mode {
                            /* per ask (pm_auction.cuh); no reference counterpart, self-oracle */
 };
 enum pm_path {
-  PM_PATH_MATERIALIZED = 0,      /* build int64 cost tile in HBM, then argmin over it */
+  PM_PATH_MATERIALIZED = 0,      /* build a cost tile in HBM, then argmin over it: 16-bit price words when every */
+                                 /* ext_ask_price <= 0xFFFE and the fast predicate applies, else int64 keys    */
   PM_PATH_FUSED        = 1u << 8,/* evaluate + reduce on chip, matrix never written   */
   PM_NO_ASK_STATS      = 1u << 9 /* with PM_PATH_FUSED: skip ask_best / ask_count (the reference modes only
                                     need the per-worker first feasible ask); they read INF / 0 then      */
@@ -254,7 +255,7 @@ enum pm_path {
 
 typedef struct pm_stats {
   uint64_t evals;            /* predicate evaluations executed on the device        */
-  uint64_t cost_bytes_written;
+  uint64_t cost_bytes_written; /* materialised path: 2 (16-bit tile) or 8 (int64 tile) B per evaluation */
   uint64_t cost_bytes_read;
   uint32_t n_tiles;          /* cost tiles; auction mode: class (re)scans           */
   uint32_t n_launches;       /* kernels of this library launched by the last match  */

@@ -149,6 +149,7 @@ struct pm_engine {
   uint32_t max_pattern_row = 0;
   bool have_workers = false, have_asks = false, have_bits = false, have_loc = false, have_rank = false;
   bool all_solo = true;  // every ask has min == max == 1
+  int tune_cost = 0;   // PM_TUNE_COST=8: the int64 cost tile even where 16-bit price words would do (in-binary A/B)
   int tune_argmin = 0, tune_generic = 0, tune_build = 0, tune_auction = 0, tune_prox = 0, tune_auc_good = 0, tune_auc_extra = 0;   // PM_TUNE_ARGMIN: kernel-shape experiments (see profiles/)
   DevBuf<uint4> wa, wb;
   DevBuf<double> lat, lon;
@@ -167,6 +168,7 @@ struct pm_engine {
   bool asks_small = true;      // every ask operand fits the fast predicate (pm_device.cuh DevOptF)
   bool workers_small = false;  // ... and every worker operand (checked on the device)
   bool workers_checked = false;
+  bool prices_narrow = false;  // every ext_ask_price <= 0xFFFE: the cost tile can hold 16-bit price words (same check)
   DevBuf<uint32_t> amin, amax, bits;
   DevBuf<uint32_t> scratch_idx, scratch_flags;
   DevBuf<uint4> upd_a, upd_b;          // staging of pm_update_workers
@@ -174,7 +176,7 @@ struct pm_engine {
   uint64_t table_version = 0;          // bumped by every call that changes a table (pm_table_version)
 
   // evaluation
-  DevBuf<long long> cost;
+  DevBuf<unsigned char> cost;   // the materialised cost tile (int64 keys or 16-bit price words), sized in bytes
   DevBuf<uint32_t> first_ask, ask_count;
   DevBuf<long long> ask_best;
 
@@ -383,6 +385,7 @@ int pm_create(const pm_cfg* cfg, pm_engine** out) try {
   if (const char* t = std::getenv("PM_TUNE_ARGMIN")) e->tune_argmin = std::atoi(t);
   if (const char* t = std::getenv("PM_TUNE_GENERIC")) e->tune_generic = std::atoi(t);
   if (const char* t = std::getenv("PM_TUNE_BUILD")) e->tune_build = std::atoi(t);
+  if (const char* t = std::getenv("PM_TUNE_COST")) e->tune_cost = std::atoi(t);
   if (const char* t = std::getenv("PM_TUNE_AUCTION")) e->tune_auction = std::atoi(t);
   if (const char* t = std::getenv("PM_TUNE_AUCTION_POOL")) std::sscanf(t, "%d,%d", &e->tune_auc_good, &e->tune_auc_extra);   // pool fill of a class walk
   if (const char* t = std::getenv("PM_TUNE_PROX")) e->tune_prox = std::atoi(t);   // 0: all-SM cooperative sweep; 2: single-CTA sweep; 1: latitude-banded single-CTA sweep (experimental)
@@ -726,15 +729,17 @@ static int decide_fast(pm_engine* e, bool* fast) {
   *fast = false;
   if (e->tune_generic || !e->asks_small) return PM_OK;
   if (!e->workers_checked) {
-    uint32_t one = 1;
-    PM_CUDA(cudaMemcpyAsync(e->counters.p + 2, &one, 4, cudaMemcpyHostToDevice, e->stream));
+    static const uint32_t ones[2] = {1u, 1u};
+    PM_CUDA(cudaMemcpyAsync(e->counters.p + 2, ones, 8, cudaMemcpyHostToDevice, e->stream));
     if (e->n_workers) {
-      pm::pm_check_worker_ranges<<<blocks_for(e->n_workers, 256), 256, 0, e->stream>>>(e->wa.p, e->wb.p, e->n_workers, e->counters.p + 2);
+      pm::pm_check_worker_ranges<<<blocks_for(e->n_workers, 256), 256, 0, e->stream>>>(e->wa.p, e->wb.p, e->n_workers, e->counters.p + 2,
+                                                                                       e->counters.p + 3);
       PM_LAUNCH_CHECK("pm_check_worker_ranges");
     }
-    PM_CUDA(cudaMemcpyAsync(e->h_scalars.p + 4, e->counters.p + 2, 4, cudaMemcpyDeviceToHost, e->stream));
+    PM_CUDA(cudaMemcpyAsync(e->h_scalars.p + 4, e->counters.p + 2, 8, cudaMemcpyDeviceToHost, e->stream));
     PM_CUDA(cudaStreamSynchronize(e->stream));
     e->workers_small = e->h_scalars.p[4] != 0;
+    e->prices_narrow = e->h_scalars.p[5] != 0;
     e->workers_checked = true;
   }
   *fast = e->workers_small;
@@ -779,33 +784,52 @@ static int worker_major(pm_engine* e, pm::EvalParams* p, int* bits_mode) {
   return PM_OK;
 }
 
-static void launch_build(pm_engine* e, const pm::EvalParams& p, int bits_mode, bool fast, dim3 grid,
-                         uint32_t t0, uint32_t nt, uint32_t w0, uint32_t nw, size_t ld) {
-#define PM_BUILD_CASE(B, F) pm::pm_build_cost<B, F><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld)
+// Does launch_build run the FastRow kernel (pm_build_cost_fast) for this table shape?  Only that kernel has the 16-bit
+// form; PM_TUNE_BUILD=1 (staged-CSR kernel) and, with one-word acceptance rows, 3 / 4 (its occupancy variants) keep int64.
+static bool fastrow_build(const pm_engine* e, bool fast, int bits_mode) {
+  return fast && e->tune_build != 1 && !(bits_mode == 2 && (e->tune_build == 3 || e->tune_build == 4));
+}
+
+// The cost tile holds 16-bit price words (2 B per evaluation instead of 8) when the FastRow kernel runs and every worker
+// price fits below the infeasible word 0xFFFF (decide_fast checked it); PM_TUNE_COST=8 forces the int64 tile.
+static bool narrow_cost(const pm_engine* e, bool fast, int bits_mode) {
+  return fastrow_build(e, fast, bits_mode) && e->prices_narrow && e->tune_cost != 8;
+}
+
+// `tile`: nt rows of ld words, int64 keys or (narrow) 16-bit price words
+static void launch_build(pm_engine* e, const pm::EvalParams& p, int bits_mode, bool fast, bool narrow, dim3 grid,
+                         uint32_t t0, uint32_t nt, uint32_t w0, uint32_t nw, size_t ld, void* tile) {
+  long long* const cost = static_cast<long long*>(tile);
+  uint16_t* const cost16 = static_cast<uint16_t*>(tile);
+#define PM_BUILD_CASE(B, F) pm::pm_build_cost<B, F><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, cost, ld)
+#define PM_FAST_CASE(B, R)                                                                                           \
+  if (narrow) pm::pm_build_cost_fast<B, R, uint16_t><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, cost16, ld); \
+  else pm::pm_build_cost_fast<B, R><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, cost, ld)
   if (fast && bits_mode == 2 && e->tune_build == 3) {
-    pm::pm_build_cost<2, true, 3><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
+    pm::pm_build_cost<2, true, 3><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, cost, ld);
   } else if (fast && bits_mode == 2 && e->tune_build == 4) {
-    pm::pm_build_cost<2, true, 4><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
+    pm::pm_build_cost<2, true, 4><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, cost, ld);
   } else if (fast && e->tune_build != 1) {   // the round-2 kernel; PM_TUNE_BUILD=1 keeps the staged-CSR form for A/B runs
     // one-word acceptance rows are bound into the FastRows (pm_bind_rows) however many rows there are
     if (p.words == 1) bits_mode = 2;
     if (bits_mode == 2 && e->tune_build == 5) {          // rows-per-CTA experiments (profiles/)
       grid.y = blocks_for(nt, 128);
-      pm::pm_build_cost_fast<2, 128><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
+      PM_FAST_CASE(2, 128);
     } else if (bits_mode == 2 && e->tune_build == 6) {
       grid.y = blocks_for(nt, 256);
-      pm::pm_build_cost_fast<2, 256><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
+      PM_FAST_CASE(2, 256);
     } else {
       grid.y = blocks_for(nt, pm::kFastRows);
-      if (bits_mode == 2) pm::pm_build_cost_fast<2><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
-      else if (bits_mode == 1) pm::pm_build_cost_fast<1><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
-      else pm::pm_build_cost_fast<0><<<grid, pm::kEvalThreads, 0, e->stream>>>(p, t0, nt, w0, nw, e->cost.p, ld);
+      if (bits_mode == 2) { PM_FAST_CASE(2, pm::kFastRows); }
+      else if (bits_mode == 1) { PM_FAST_CASE(1, pm::kFastRows); }
+      else { PM_FAST_CASE(0, pm::kFastRows); }
     }
   } else if (fast) {
     if (bits_mode == 2) PM_BUILD_CASE(2, true); else if (bits_mode == 1) PM_BUILD_CASE(1, true); else PM_BUILD_CASE(0, true);
   } else {
     if (bits_mode == 2) PM_BUILD_CASE(2, false); else if (bits_mode == 1) PM_BUILD_CASE(1, false); else PM_BUILD_CASE(0, false);
   }
+#undef PM_FAST_CASE
 #undef PM_BUILD_CASE
 }
 
@@ -821,12 +845,31 @@ static void launch_fused(pm_engine* e, const pm::EvalParams& p, int bits_mode, b
 #undef PM_FUSED_CASE
 }
 
-static void launch_argmin(pm_engine* e, size_t ld, uint32_t nt, uint32_t t0, uint32_t w0, uint32_t nw) {
+static void launch_argmin(pm_engine* e, bool narrow, size_t ld, uint32_t nt, uint32_t t0, uint32_t w0, uint32_t nw) {
+#define PM_ARGMIN16_CASE(S, RPW)                                                                                      \
+  {                                                                                                                   \
+    dim3 grid(blocks_for(ld, (S) * 256 * pm::kArgWarps), blocks_for(nt, pm::kArgRows));                               \
+    pm::pm_argmin16<S, RPW><<<grid, pm::kArgThreads, 0, e->stream>>>(reinterpret_cast<const uint16_t*>(e->cost.p), ld, \
+                                                                     nt, t0, w0, nw, e->first_ask.p, e->ask_best.p,  \
+                                                                     e->ask_count.p);                                 \
+  }
+  if (narrow) {   // PM_TUNE_ARGMIN picks the shape of the 16-bit kernel here (profiles/r03_argmin16_shapes.txt)
+    switch (e->tune_argmin) {
+      case 1: PM_ARGMIN16_CASE(2, 4) break;
+      case 2: PM_ARGMIN16_CASE(4, 1) break;
+      case 3: PM_ARGMIN16_CASE(8, 1) break;
+      case 4: PM_ARGMIN16_CASE(4, 4) break;
+      case 5: PM_ARGMIN16_CASE(8, 2) break;
+      default: PM_ARGMIN16_CASE(4, 2) break;
+    }
+    return;
+  }
+#undef PM_ARGMIN16_CASE
 #define PM_ARGMIN_CASE(S, RPW)                                                                      \
   {                                                                                                  \
     dim3 grid(blocks_for(ld, (S) * 64 * pm::kArgWarps), blocks_for(nt, pm::kArgRows));                               \
-    pm::pm_argmin<S, RPW><<<grid, pm::kArgThreads, 0, e->stream>>>(e->cost.p, ld, nt, t0, w0, nw,    \
-                                                                   e->first_ask.p, e->ask_best.p,   \
+    pm::pm_argmin<S, RPW><<<grid, pm::kArgThreads, 0, e->stream>>>(reinterpret_cast<const long long*>(e->cost.p), ld, \
+                                                                   nt, t0, w0, nw, e->first_ask.p, e->ask_best.p,    \
                                                                    e->ask_count.p);                 \
   }
   switch (e->tune_argmin) {
@@ -916,12 +959,17 @@ static int match_local_locked(pm_engine* e, uint32_t mode) {
         const int rc = bind_rows(e, wm);
         if (rc != PM_OK) return rc;
       }
+      const bool narrow = narrow_cost(e, fast, bits_mode);
+      const size_t word_bytes = narrow ? 2 : 8;    // 16-bit price words or int64 keys
+      // rows per tile as the int64 tile has them, whatever the width: both widths run the same tile sequence (the A/B
+      // differs in the word alone) and the 16-bit tile takes a quarter of the budget.  Taller 16-bit tiles were faster on
+      // cfg3 (4096 rows: 7 %, profiles/r03_cost_width_ab_4096_rows.txt)
       uint64_t rows = e->cfg.cost_tile_bytes / (ld * 8);
       if (rows == 0) rows = 1;
       rows = std::min<uint64_t>(rows, T);
       rows = std::min<uint64_t>(rows, 65535ull * pm::kArgRows);
       if (rows >= 1024) rows &= ~(uint64_t)511;   // whole row bands of the build kernel (no ragged last band in every tile)
-      cudaError_t ce = e->cost.ensure((size_t)rows * ld);
+      cudaError_t ce = e->cost.ensure((size_t)rows * ld * word_bytes);
       if (ce != cudaSuccess) {
         cudaGetLastError();
         return e->fail(PM_E_NOMEM, "pm_match: cannot allocate the cost tile; lower pm_cfg.cost_tile_bytes");
@@ -931,21 +979,22 @@ static int match_local_locked(pm_engine* e, uint32_t mode) {
         {
           Timer tm(e, &e->stats.ms_build);
           dim3 grid(blocks_for(ld, pm::kEvalCols), blocks_for(nt, pm::kEvalRows));
-          launch_build(e, p, bits_mode, fast, grid, t0, nt, w0, nw, ld);
+          launch_build(e, p, bits_mode, fast, narrow, grid, t0, nt, w0, nw, ld, e->cost.p);
           PM_LAUNCH_CHECK("pm_build_cost");
           tm.stop();
           ++e->stats.n_build_launches;
         }
         {
           Timer tm(e, &e->stats.ms_argmin);
-          launch_argmin(e, ld, nt, t0, w0, nw);
+          launch_argmin(e, narrow, ld, nt, t0, w0, nw);
           PM_LAUNCH_CHECK("pm_argmin");
           tm.stop();
           ++e->stats.n_argmin_launches;
         }
         ++e->stats.n_tiles;
-        e->stats.cost_bytes_written += (uint64_t)nt * nw * 8;   // algorithmic: 8 B per evaluation (padding columns not counted)
-        e->stats.cost_bytes_read += (uint64_t)nt * nw * 8;
+        // algorithmic: 2 or 8 B per evaluation (padding columns not counted)
+        e->stats.cost_bytes_written += (uint64_t)nt * nw * word_bytes;
+        e->stats.cost_bytes_read += (uint64_t)nt * nw * word_bytes;
       }
     }
     e->stats.evals = (uint64_t)T * nw;
@@ -1630,10 +1679,6 @@ int pm_build_cost_tile(pm_engine* e, uint32_t t0, uint32_t nt, int64_t* host_out
   }
   const size_t ld = (((size_t)nw + pm::kEvalCols - 1) / pm::kEvalCols) * pm::kEvalCols;
   if (nt > 65535u * pm::kEvalRows) return e->fail(PM_E_INVALID, "pm_build_cost_tile: too many rows");
-  if (e->cost.ensure((size_t)nt * ld) != cudaSuccess) {
-    cudaGetLastError();
-    return e->fail(PM_E_NOMEM, "pm_build_cost_tile: cannot allocate the tile");
-  }
   pm::EvalParams p = eval_params(e);
   dim3 grid(blocks_for(ld, pm::kEvalCols), blocks_for(nt, pm::kEvalRows));
   bool fast = false;
@@ -1649,8 +1694,23 @@ int pm_build_cost_tile(pm_engine* e, uint32_t t0, uint32_t nt, int64_t* host_out
     rc = bind_rows(e, wm);
     if (rc != PM_OK) return rc;
   }
-  launch_build(e, p, bits_mode, fast, grid, t0, nt, w0, nw, ld);
-  PM_LAUNCH_CHECK("pm_build_cost");
+  // the kernel pm_match would run: with 16-bit words the tile goes after the int64 one and is widened into it
+  const bool narrow = narrow_cost(e, fast, bits_mode);
+  const size_t wide_bytes = (size_t)nt * ld * 8;
+  if (e->cost.ensure(wide_bytes + (narrow ? (size_t)nt * ld * 2 : 0)) != cudaSuccess) {
+    cudaGetLastError();
+    return e->fail(PM_E_NOMEM, "pm_build_cost_tile: cannot allocate the tile");
+  }
+  if (narrow) {
+    launch_build(e, p, bits_mode, fast, true, grid, t0, nt, w0, nw, ld, e->cost.p + wide_bytes);
+    PM_LAUNCH_CHECK("pm_build_cost");
+    pm::pm_widen_cost<<<std::min(blocks_for((size_t)nt * ld, 256), 4096u), 256, 0, e->stream>>>(
+        reinterpret_cast<const uint16_t*>(e->cost.p + wide_bytes), (size_t)nt * ld, ld, w0, reinterpret_cast<long long*>(e->cost.p));
+    PM_LAUNCH_CHECK("pm_widen_cost");
+  } else {
+    launch_build(e, p, bits_mode, fast, false, grid, t0, nt, w0, nw, ld, e->cost.p);
+    PM_LAUNCH_CHECK("pm_build_cost");
+  }
   PM_CUDA(cudaMemcpy2DAsync(host_out, (size_t)nw * 8, e->cost.p, ld * 8, (size_t)nw * 8, nt,
                             cudaMemcpyDeviceToHost, e->stream));
   PM_CUDA(cudaStreamSynchronize(e->stream));

@@ -1,9 +1,12 @@
 // pm_kernels.cuh — sm_100a kernels of the matching pass.
 //
 //   pm_build_cost   cost-matrix build: int64 cost[t][w] for a tile of asks x a
-//                   stripe of workers, HBM-write-bound (8 B per evaluation)
+//                   stripe of workers, HBM-write-bound (8 B per evaluation);
+//                   pm_build_cost_fast<.., uint16_t> writes 16-bit price words
+//                   (2 B per evaluation) when every worker price is <= 0xFFFE
 //   pm_argmin       one read of the tile (8 B per evaluation): per-ask packed
-//                   (min_cost, argmin) + feasible count, per-worker first ask
+//                   (min_cost, argmin) + feasible count, per-worker first ask;
+//                   pm_argmin16 the same from a 16-bit tile (2 B per evaluation)
 //   pm_fused_eval   the same outputs without materialising the matrix
 //   pm_hist / pm_check_tails / pm_sweep / pm_emit_* : resolution sweep that turns
 //                   "first feasible ask per worker" into the reference's groups
@@ -348,66 +351,136 @@ struct __align__(128) FastStage {
 constexpr int kFastRows = 512;   // asks per CTA: the prologue (worker rows from L2, the TMA of the FastRows) is paid once per CTA
                                  // (measured on cfg3: 128 rows 119.1 ms/step, 256 rows 116.3, 512 rows 113.8 — profiles/r02_build_rows.txt)
 
-template <int BITS, int ROWS = kFastRows>
-__global__ void __launch_bounds__(kEvalThreads, 2)
-pm_build_cost_fast(EvalParams p, uint32_t t0, uint32_t nt, uint32_t w0, uint32_t nw, long long* __restrict__ cost, size_t ld) {
-  __shared__ FastStage<ROWS> s;
-  const uint32_t r0 = blockIdx.y * ROWS;
-  const uint32_t nrows = min(nt - r0, (uint32_t)ROWS);
-  if (threadIdx.x == 0) {
-    mbar_init(&s.bar, 1);
-    mbar_expect_tx(&s.bar, nrows * (uint32_t)sizeof(FastRow));
-    bulk_g2s(s.row, p.frows + t0 + r0, nrows * (uint32_t)sizeof(FastRow), &s.bar);
-  }
-  if (BITS == 1) {
-    const uint32_t total_words = p.n_bits_rows * p.words;
-    for (uint32_t i = threadIdx.x; i < total_words; i += blockDim.x) s.bits[i] = __ldg(p.bits + i);
-  }
-  const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t cbase = blockIdx.x * kEvalCols + (threadIdx.x >> 5) * 128u + lane * 2u;
-  WorkerReg w[kEvalWPT];
-  uint32_t gw[kEvalWPT], dx[kEvalWPT], dy[kEvalWPT];
-#pragma unroll
-  for (int k = 0; k < kEvalWPT; ++k) {
-    const uint32_t col = cbase + (k >> 1) * 64u + (k & 1);
-    gw[k] = w0 + col;
-    if (col < nw) {
-      w[k] = make_worker(__ldg(p.wa + w0 + col), __ldg(p.wb + w0 + col));
-      if (p.nacc) w[k].mmask = __ldg(p.nacc + w0 + col);
-    } else w[k] = null_worker();
-    dx[k] = 0xFFFFFFFFu - gw[k];          // infeasible: 0x7FFFFFFF_FFFFFFFF = feasible word + (0/1) * difference
-    dy[k] = 0x7FFFFFFFu - w[k].price;
-  }
-  uint4* out = reinterpret_cast<uint4*>(cost + (size_t)r0 * ld + cbase);
-  const size_t row_stride = ld / 2;
-  const uint32_t sh = p.sign_shift;
-  __syncthreads();            // mbarrier initialised, acceptance words staged
-  mbar_wait(&s.bar, 0);
-  FastRow cur = s.row[0];
-  for (uint32_t r = 0; r < nrows; ++r) {
-    FastRow nxt = cur;
-    if (r + 1 < nrows) nxt = s.row[r + 1];    // in flight while this row is evaluated
-    uint32_t um[kEvalWPT];
-    eval_fast_first<kEvalWPT, BITS>(cur, s.bits, w, p.bits, p.words, um);
-    if (cur.n_opts > 1u)                      // OR-options (node.rs:420-438): the ask fails only if every option does
-      eval_fast_more<kEvalWPT, BITS>(p.opts_fast + cur.opt_off + 1, cur.n_opts - 1u, s.bits, w, p.bits, p.words, um);
-    uint4 v0, v1;
-    {
-      uint32_t o[2 * kEvalWPT];
-#pragma unroll
-      for (int k = 0; k < kEvalWPT; ++k) {
-        const uint32_t fail = um[k] | (w[k].cores - cur.cpu_cores) | (w[k].ram - cur.ram_mb) | (w[k].storage - cur.storage_gb);
-        const uint32_t b = fail >> sh;                                    // 1 when infeasible (sh == 31)
-        o[2 * k] = b * dx[k] + gw[k];                                     // feasible: (price << 32) | worker
-        o[2 * k + 1] = b * dy[k] + w[k].price;                            // infeasible: 0x7FFFFFFF_FFFFFFFF
-      }
-      v0 = make_uint4(o[0], o[1], o[2], o[3]);
-      v1 = make_uint4(o[4], o[5], o[6], o[7]);
+// Word = long long: the int64 packed cost (price << 32 | worker, 0x7FFFFFFF_FFFFFFFF when infeasible), 8 B per
+// evaluation; a lane owns the column pairs (2l, 2l+1) and (64+2l, 64+2l+1) of its warp's 128 columns (two 128-bit stores
+// per row).  Word = uint16_t: the price word (price, 0xFFFF when infeasible), 2 B per evaluation, for worker tables whose
+// prices are all <= 0xFFFE — the worker index is the column, so the word carries everything the argmin needs; a lane
+// owns 4 consecutive columns and writes them with one 64-bit store per row (a warp 256 B contiguous).
+template <int BITS, int ROWS = kFastRows, typename Word = long long, int MINB = 2>
+__global__ void __launch_bounds__(kEvalThreads, MINB)
+pm_build_cost_fast(EvalParams p, uint32_t t0, uint32_t nt, uint32_t w0, uint32_t nw, Word* __restrict__ cost, size_t ld) {
+  static_assert(sizeof(Word) == 2 || sizeof(Word) == 8, "cost word is int64 or 16-bit");
+  if constexpr (sizeof(Word) == 2) {
+    __shared__ FastStage<ROWS> s;
+    const uint32_t r0 = blockIdx.y * ROWS;
+    const uint32_t nrows = min(nt - r0, (uint32_t)ROWS);
+    if (threadIdx.x == 0) {
+      mbar_init(&s.bar, 1);
+      mbar_expect_tx(&s.bar, nrows * (uint32_t)sizeof(FastRow));
+      bulk_g2s(s.row, p.frows + t0 + r0, nrows * (uint32_t)sizeof(FastRow), &s.bar);
     }
-    __stcs(out, v0);
-    __stcs(out + 32, v1);     // + 64 columns
-    out += row_stride;
-    cur = nxt;
+    if (BITS == 1) {
+      const uint32_t total_words = p.n_bits_rows * p.words;
+      for (uint32_t i = threadIdx.x; i < total_words; i += blockDim.x) s.bits[i] = __ldg(p.bits + i);
+    }
+    const uint32_t cbase = blockIdx.x * kEvalCols + threadIdx.x * 4u;   // 4 consecutive columns per lane
+    WorkerReg w[kEvalWPT];
+    // word = price + b * (0xFFFF - price), two words per 32-bit half of the store.  The odd column's difference is
+    // pre-shifted and both prices pre-packed, so a half is two multiply-adds: b1 * (d1 << 16) + (b0 * d0 + (p0 | p1 << 16));
+    // b0 * d0 + p0 <= 0xFFFF, so nothing carries into the upper word.  Padding columns are null workers: 0xFFFF.
+    uint32_t nd[kEvalWPT];
+#pragma unroll
+    for (int k = 0; k < kEvalWPT; ++k) {
+      const uint32_t col = cbase + k;
+      if (col < nw) {
+        w[k] = make_worker(__ldg(p.wa + w0 + col), __ldg(p.wb + w0 + col));
+        if (p.nacc) w[k].mmask = __ldg(p.nacc + w0 + col);
+      } else w[k] = null_worker();
+      nd[k] = (0xFFFFu - w[k].price) << ((k & 1) * 16);
+    }
+    const uint32_t np0 = w[0].price | (w[1].price << 16), np1 = w[2].price | (w[3].price << 16);
+    uint2* out = reinterpret_cast<uint2*>(cost + (size_t)r0 * ld + cbase);
+    const size_t row_stride = ld / 4;   // in 8-byte units
+    const uint32_t sh = p.sign_shift;
+    __syncthreads();
+    mbar_wait(&s.bar, 0);
+    FastRow cur = s.row[0];
+    for (uint32_t r = 0; r < nrows; ++r) {
+      FastRow nxt = cur;
+      if (r + 1 < nrows) nxt = s.row[r + 1];
+      uint32_t um[kEvalWPT];
+      eval_fast_first<kEvalWPT, BITS>(cur, s.bits, w, p.bits, p.words, um);
+      if (cur.n_opts > 1u)
+        eval_fast_more<kEvalWPT, BITS>(p.opts_fast + cur.opt_off + 1, cur.n_opts - 1u, s.bits, w, p.bits, p.words, um);
+      uint32_t b[kEvalWPT];
+#pragma unroll
+      for (int k = 0; k < kEvalWPT; ++k)
+        b[k] = (um[k] | (w[k].cores - cur.cpu_cores) | (w[k].ram - cur.ram_mb) | (w[k].storage - cur.storage_gb)) >> sh;
+      uint2 v;
+      v.x = b[1] * nd[1] + (b[0] * nd[0] + np0);
+      v.y = b[3] * nd[3] + (b[2] * nd[2] + np1);
+      __stcs(out, v);
+      out += row_stride;
+      cur = nxt;
+    }
+  } else {
+    __shared__ FastStage<ROWS> s;
+    const uint32_t r0 = blockIdx.y * ROWS;
+    const uint32_t nrows = min(nt - r0, (uint32_t)ROWS);
+    if (threadIdx.x == 0) {
+      mbar_init(&s.bar, 1);
+      mbar_expect_tx(&s.bar, nrows * (uint32_t)sizeof(FastRow));
+      bulk_g2s(s.row, p.frows + t0 + r0, nrows * (uint32_t)sizeof(FastRow), &s.bar);
+    }
+    if (BITS == 1) {
+      const uint32_t total_words = p.n_bits_rows * p.words;
+      for (uint32_t i = threadIdx.x; i < total_words; i += blockDim.x) s.bits[i] = __ldg(p.bits + i);
+    }
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t cbase = blockIdx.x * kEvalCols + (threadIdx.x >> 5) * 128u + lane * 2u;
+    WorkerReg w[kEvalWPT];
+    uint32_t gw[kEvalWPT], dx[kEvalWPT], dy[kEvalWPT];
+  #pragma unroll
+    for (int k = 0; k < kEvalWPT; ++k) {
+      const uint32_t col = cbase + (k >> 1) * 64u + (k & 1);
+      gw[k] = w0 + col;
+      if (col < nw) {
+        w[k] = make_worker(__ldg(p.wa + w0 + col), __ldg(p.wb + w0 + col));
+        if (p.nacc) w[k].mmask = __ldg(p.nacc + w0 + col);
+      } else w[k] = null_worker();
+      dx[k] = 0xFFFFFFFFu - gw[k];          // infeasible: 0x7FFFFFFF_FFFFFFFF = feasible word + (0/1) * difference
+      dy[k] = 0x7FFFFFFFu - w[k].price;
+    }
+    uint4* out = reinterpret_cast<uint4*>(cost + (size_t)r0 * ld + cbase);
+    const size_t row_stride = ld / 2;
+    const uint32_t sh = p.sign_shift;
+    __syncthreads();            // mbarrier initialised, acceptance words staged
+    mbar_wait(&s.bar, 0);
+    FastRow cur = s.row[0];
+    for (uint32_t r = 0; r < nrows; ++r) {
+      FastRow nxt = cur;
+      if (r + 1 < nrows) nxt = s.row[r + 1];    // in flight while this row is evaluated
+      uint32_t um[kEvalWPT];
+      eval_fast_first<kEvalWPT, BITS>(cur, s.bits, w, p.bits, p.words, um);
+      if (cur.n_opts > 1u)                      // OR-options (node.rs:420-438): the ask fails only if every option does
+        eval_fast_more<kEvalWPT, BITS>(p.opts_fast + cur.opt_off + 1, cur.n_opts - 1u, s.bits, w, p.bits, p.words, um);
+      uint4 v0, v1;
+      {
+        uint32_t o[2 * kEvalWPT];
+  #pragma unroll
+        for (int k = 0; k < kEvalWPT; ++k) {
+          const uint32_t fail = um[k] | (w[k].cores - cur.cpu_cores) | (w[k].ram - cur.ram_mb) | (w[k].storage - cur.storage_gb);
+          const uint32_t b = fail >> sh;                                    // 1 when infeasible (sh == 31)
+          o[2 * k] = b * dx[k] + gw[k];                                     // feasible: (price << 32) | worker
+          o[2 * k + 1] = b * dy[k] + w[k].price;                            // infeasible: 0x7FFFFFFF_FFFFFFFF
+        }
+        v0 = make_uint4(o[0], o[1], o[2], o[3]);
+        v1 = make_uint4(o[4], o[5], o[6], o[7]);
+      }
+      __stcs(out, v0);
+      __stcs(out + 32, v1);     // + 64 columns
+      out += row_stride;
+      cur = nxt;
+    }
+  }
+}
+
+// The int64 packed cost of a 16-bit tile (pm_build_cost_tile's host output): price << 32 | worker, or
+// 0x7FFFFFFF_FFFFFFFF where the word is 0xFFFF.
+__global__ void pm_widen_cost(const uint16_t* __restrict__ in, size_t n, size_t ld, uint32_t w0, long long* __restrict__ out) {
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    const uint32_t h = in[i];
+    out[i] = h == 0xFFFFu ? kInf : (long long)(((unsigned long long)h << 32) | (w0 + (uint32_t)(i % ld)));
   }
 }
 
@@ -517,6 +590,105 @@ pm_argmin(const long long* __restrict__ cost, size_t ld, uint32_t nt, uint32_t t
   for (uint32_t i = threadIdx.x; i < rows; i += kArgThreads) {
     if (s_cnt[i]) {
       atomicMin(ask_best + t0 + r0 + i, (long long)s_best[i]);
+      atomicAdd(ask_count + t0 + r0 + i, s_cnt[i]);
+    }
+  }
+}
+
+// 16-bit form: one read of a price-word tile (2 B per evaluation), same outputs as pm_argmin.  A lane loads 8 columns per
+// 128-bit load, S loads per row (a warp covers S*256 columns, a CTA 8*S*256 <= 65536).  The row minimum is folded on a
+// 32-bit key price << 16 | column offset: inside a lane the offset is the compile-time position of the column among the
+// lane's own (one IMAD forms the key of the low word, one LOP3 that of the high word), the lane's base offset within the
+// CTA's span is added once per row, and the key is widened to the int64 key (price << 32 | worker) only at the per-CTA
+// flush.  Infeasible words (0xFFFF) give keys >= 0xFFFF0000 and are neither counted nor folded into first_ask.
+template <int S, int RPW>
+__global__ void __launch_bounds__(kArgThreads)
+pm_argmin16(const uint16_t* __restrict__ cost, size_t ld, uint32_t nt, uint32_t t0, uint32_t w0,
+            uint32_t nw, uint32_t* __restrict__ first_ask, long long* __restrict__ ask_best,
+            uint32_t* __restrict__ ask_count) {
+  constexpr uint32_t kWarpCols = S * 256;
+  constexpr uint32_t kCtaCols = kArgWarps * kWarpCols;
+  static_assert(kCtaCols <= 65536u, "column offsets are 16 bits");
+  constexpr uint32_t kInfeasible = 0xFFFF0000u;   // keys at or above: infeasible words
+  __shared__ uint32_t s_best[kArgRows];
+  __shared__ uint32_t s_cnt[kArgRows];
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  const uint32_t cta_c0 = blockIdx.x * kCtaCols;
+  const uint32_t lane_off = warp * kWarpCols + lane * 8u;    // this lane's first column, relative to the CTA's span
+  const uint32_t c0 = cta_c0 + lane_off;
+  const uint32_t r0 = blockIdx.y * kArgRows;
+  const uint32_t rows = min((uint32_t)kArgRows, nt - r0);
+  for (uint32_t i = threadIdx.x; i < (uint32_t)kArgRows; i += kArgThreads) {
+    s_best[i] = kNone;
+    s_cnt[i] = 0;
+  }
+  __syncthreads();
+
+  uint32_t cm[S][8];
+#pragma unroll
+  for (int s = 0; s < S; ++s)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) cm[s][j] = kNone;
+
+  if (cta_c0 + warp * kWarpCols < ld) {
+    for (uint32_t rr = 0; rr < rows; rr += RPW) {
+      uint4 v[RPW][S];
+#pragma unroll
+      for (int q = 0; q < RPW; ++q) {
+        const uint4* rowp = reinterpret_cast<const uint4*>(cost + (size_t)(r0 + rr + q) * ld);
+#pragma unroll
+        for (int s = 0; s < S; ++s) {
+          const uint32_t col = c0 + s * 256;
+          if (rr + q < rows && col < ld) v[q][s] = __ldcs(rowp + (col >> 3));
+          else v[q][s] = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
+        }
+      }
+#pragma unroll
+      for (int q = 0; q < RPW; ++q) {
+        const uint32_t t = t0 + r0 + rr + q;
+        uint32_t best = kInfeasible, cnt = 0;
+#pragma unroll
+        for (int s = 0; s < S; ++s) {
+          const uint32_t x4[4] = {v[q][s].x, v[q][s].y, v[q][s].z, v[q][s].w};
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const uint32_t x = x4[j];
+            const uint32_t off = s * 256 + 2 * j;             // lane-relative: s * 256 + 2j (+ 1 for the high word)
+            const uint32_t klo = x * 65536u + off;            // (low word << 16) | off
+            const uint32_t khi = (x & 0xFFFF0000u) | (off + 1u);
+            best = min(best, min(klo, khi));                  // strict order: the lower column wins a tie in price
+            const bool flo = klo < kInfeasible, fhi = x < kInfeasible;
+            cnt += (uint32_t)flo + (uint32_t)fhi;
+            cm[s][2 * j] = flo ? min(cm[s][2 * j], t) : cm[s][2 * j];
+            cm[s][2 * j + 1] = fhi ? min(cm[s][2 * j + 1], t) : cm[s][2 * j + 1];
+          }
+        }
+        best += lane_off;                                     // < 0xFFFF0000 + 65536: no carry out of the key
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
+          cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+        }
+        if (lane == 0 && cnt) {
+          atomicMin(&s_best[rr + q], best);
+          atomicAdd(&s_cnt[rr + q], cnt);
+        }
+      }
+    }
+#pragma unroll
+    for (int s = 0; s < S; ++s)
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const uint32_t col = c0 + s * 256 + j;
+        if (cm[s][j] != kNone && col < nw) atomicMin(first_ask + w0 + col, cm[s][j]);
+      }
+  }
+  __syncthreads();
+  for (uint32_t i = threadIdx.x; i < rows; i += kArgThreads) {
+    if (s_cnt[i]) {   // a counted row has a feasible minimum: key < 0xFFFF0000
+      const uint32_t key = s_best[i];
+      const unsigned long long wide = ((unsigned long long)(key >> 16) << 32) | (w0 + cta_c0 + (key & 0xFFFFu));
+      atomicMin(ask_best + t0 + r0 + i, (long long)wide);
       atomicAdd(ask_count + t0 + r0 + i, s_cnt[i]);
     }
   }
@@ -747,9 +919,10 @@ __global__ void pm_scatter_rows(uint4* wa, uint4* wb, double* lat, double* lon, 
 }
 
 // Do all workers satisfy the fast-path operand limits (values < 2^31, gpu count < 2^16,
-// count * memory_mb < 2^31 without wrapping)?  Clears *ok otherwise.
+// count * memory_mb < 2^31 without wrapping)?  Clears *ok otherwise.  Clears *narrow when a
+// worker's ext_ask_price does not fit a 16-bit cost word (> 0xFFFE: 0xFFFF means infeasible).
 __global__ void pm_check_worker_ranges(const uint4* __restrict__ wa, const uint4* __restrict__ wb,
-                                       uint32_t n, uint32_t* __restrict__ ok) {
+                                       uint32_t n, uint32_t* __restrict__ ok, uint32_t* __restrict__ narrow) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const uint4 a = wa[i], b = wb[i];
@@ -759,6 +932,7 @@ __global__ void pm_check_worker_ranges(const uint4* __restrict__ wa, const uint4
   if ((a.w & PM_W_HAS_GPU_COUNT) && (a.w & PM_W_HAS_GPU_MEM))
     small &= (unsigned long long)a.x * (unsigned long long)a.y < (unsigned long long)kSign;
   if (!small) *ok = 0u;
+  if (b.w > 0xFFFEu) *narrow = 0u;
 }
 
 // ------------------------------------------------------------------ resolution
